@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — frames/s of the hybrid-ensemble inference hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--config C] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--config C] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch of B synthetic RGB frames per GPU.  `--config`:
   ensemble (default, BASELINE config 4, the workload the metric is quoted on): bilinear resize+BGR -> LM (U-Net++/
@@ -22,6 +22,10 @@ pre/post kernels), `cpu_baseline` = the CPU oracle port on host cores.
 `--impl reference` times the reference's own CPU implementation of the path restated in oracle/ (the original cannot
 be installed offline: smp/timm/efficientnet_pytorch/lightning/hydra are absent, see DESIGN.md) on all host threads,
 batch 1 per call as src/predict.py does.
+
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (mask, label, counts, radii of
+EnsemblePipeline.run_device) as DIR/<name>.npy, so that two builds run with the same arguments, and hence the same
+seeded frames and weights, can be compared output for output (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -172,6 +176,26 @@ def reference_arm(args):
     emit(line)
 
 
+DUMP_MAX_ELEMENTS = 1 << 22          # per output: 16 MB as float32, so the four outputs stay well under 64 MB
+DUMP_SEED = 0
+
+
+def dump_outputs(dst: str, outputs: dict) -> None:
+    """Each device tensor becomes dst/<name>.npy: float64 for 32/64-bit integers and float64 data, float32 otherwise
+    (both exact for these outputs).  A tensor of more than DUMP_MAX_ELEMENTS elements is stored as a sample of its
+    flattened elements: one position in each of DUMP_MAX_ELEMENTS equal strides, drawn by a generator seeded with
+    DUMP_SEED and the tensor's size, so the same shape always yields the same positions."""
+    os.makedirs(dst, exist_ok=True)
+    for name, t in outputs.items():
+        n, k = t.numel(), DUMP_MAX_ELEMENTS
+        if n > k:
+            stride = n // k
+            idx = np.arange(k, dtype=np.int64) * stride + np.random.default_rng([DUMP_SEED, n]).integers(0, stride, size=k)
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        wide = t.dtype in (torch.int32, torch.int64, torch.float64)
+        np.save(os.path.join(dst, f'{name}.npy'), t.cpu().numpy().astype(np.float64 if wide else np.float32))
+
+
 def lib_sha16() -> str:
     import hashlib
     path = os.path.join(ROOT, 'oct_segmentation_b200', 'liboctseg.so')
@@ -309,8 +333,8 @@ def ours_arm(args):
     barrier()
     e0.record()
     for i in range(K):
-        _, _, counts, _ = pipe.run_device(dev_batches[i % len(dev_batches)])
-        counts_log.append(counts.clone())
+        outputs = pipe.run_device(dev_batches[i % len(dev_batches)])
+        counts_log.append(outputs[2].clone())
     table = gather_table(torch.cat(counts_log), world * B * K) if world > 1 else torch.cat(counts_log)
     e1.record()
     barrier()
@@ -320,6 +344,8 @@ def ours_arm(args):
     t_ms = t_ms.item()
     clocks = sampler.stop() if rank == 0 else None
     value = world * B * K / (t_ms * 1e-3)
+    if args.dump_outputs and rank == 0:             # before the passes below overwrite the pipeline's output buffers
+        dump_outputs(args.dump_outputs, {k: v for k, v in zip(('mask', 'label', 'counts', 'radii'), outputs) if v is not None})
 
     # ---------------------------------------------------------------- end to end (host buffers)
     host_np = host.numpy()
@@ -515,7 +541,13 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-rooflines', action='store_true',
                     help='skip the instrumented per-launch passes (for the ncu launch list: only the timed steps run)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/<name>.npy (a seeded sample of the large ones)')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and (args.e2e_files > 0 or args.impl == 'reference'):
+        ap.error('--dump-outputs applies to the device-resident timed path (--impl ours without --e2e-files)')
     _claim_stdout()
     if args.e2e_files > 0:
         files_arm(args)

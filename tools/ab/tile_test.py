@@ -1,5 +1,5 @@
-import json, sys
-sys.path.insert(0, '/root/repo')
+import json, os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import torch
 from oct_segmentation_b200.engine import conv as C
 N = 32

@@ -1,5 +1,5 @@
 import sys, os
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from oct_segmentation_b200.model import OCTSegmentationModel
 from oct_segmentation_b200.engine.network import CompiledNet

@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define OCTSEG_ABI_VERSION 2
+#define OCTSEG_ABI_VERSION 3
 
 enum {
   OCTSEG_OK = 0,
@@ -164,26 +164,10 @@ int octseg_dwconv(const void* in, const void* weight /* bf16 [kh][kw][C] */, con
                   float* pool_sum, int32_t pool_slots, void* stream);
 int octseg_dwconv_pool_slots(int32_t C, int32_t Ho, int32_t Wo);
 
-/* Fused front half of an MBConv block (efficientnet_pytorch MBConvBlock: _expand_conv -> _bn0 -> swish ->
-   _depthwise_conv (static "same" padding) -> _bn1 -> swish, plus the squeeze-excite channel sums), BatchNorms folded.
-   Replaces one octseg_conv_run (1x1, swish) + one octseg_dwconv: the expanded tensor stays in TMEM / shared memory.
-   x: bf16 NHWC [N][H][W][ldc_in] (Cin real channels, Cin % 16 == 0); w_exp: bf16 [Cmid][Cin];
-   blob: fp32 [ceil(Cmid/64)][2 + k*k][64], per 64-channel block c0: row 0 = b_exp[c0..]/2, row 1 = b_dw[c0..]/2,
-   row 2 + ky*k + kx = w_dw[ky][kx][c0..]/2 (zero beyond Cmid; the halving is the swish form h*tanh(h)+h, h = x/2);
-   out: bf16 NHWC [N][Ho][Wo][Cmid]; k in {3,5}, stride 1; pool_sum: fp32 [N][slots][Cmid] per-tile partial sums
-   (slots = octseg_mbconv_pool_slots(k, Ho, Wo), each written once) or NULL.  EINVAL if the tile does not fit shared memory (octseg_mbconv_smem_bytes(Cin, k, stride) >
-   227 KB, or < 0 for unsupported shapes).  octseg_mbconv_blob_floats(Cmid, k) = number of floats in `blob`. */
-int octseg_mbconv_expand_dw(const void* x, int32_t N, int32_t H, int32_t W, int32_t Cin, int32_t ldc_in,
-                            const void* w_exp, const float* blob, void* out, int32_t Cmid, int32_t k, int32_t stride,
-                            int32_t pad_t, int32_t pad_l, int32_t Ho, int32_t Wo, float* pool_sum, void* stream);
-int octseg_mbconv_smem_bytes(int32_t Cin, int32_t k, int32_t stride);
-int octseg_mbconv_blob_floats(int32_t Cmid, int32_t k);
-int octseg_mbconv_pool_slots(int32_t k, int32_t Ho, int32_t Wo);
-
 /* Squeeze-excite (efficientnet_pytorch MBConvBlock: adaptive_avg_pool2d -> _se_reduce -> swish ->
    _se_expand -> sigmoid -> gate * x), folded into the projection 1x1 conv's weights:
    hidden[n][r] = swish(w1[r,:] . (sum_s pool_sum[n,s,:] * inv_hw) + b1[r])          fp32 [N][Cr]
-   pool_sum: fp32 [N][slots][C] partial sums (octseg_dwconv / octseg_mbconv_expand_dw), added in slot order into
+   pool_sum: fp32 [N][slots][C] partial sums (octseg_dwconv), added in slot order into
    sums_scratch fp32 [N][C] first (a second tiny launch; may be NULL when slots == 1). */
 int octseg_se_hidden(const float* pool_sum, int32_t slots, float* sums_scratch, float inv_hw,
                      const float* w1 /* [Cr][C] */, const float* b1, float* hidden, int32_t N, int32_t C, int32_t Cr,

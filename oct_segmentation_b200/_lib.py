@@ -24,7 +24,7 @@ EXPORTS = [
     'octseg_stem_pack', 'octseg_maxpool3x3s2', 'octseg_dwconv', 'octseg_se_hidden',
     'octseg_se_gate', 'octseg_se_scale_weights', 'octseg_preprocess_resize_bgr', 'octseg_postprocess',
     'octseg_radial_thickness', 'octseg_overlay', 'octseg_preprocess_resize_gray',
-    'octseg_fold_average_threshold', 'octseg_contour_largest', 'octseg_mbconv_expand_dw', 'octseg_mbconv_smem_bytes', 'octseg_mbconv_blob_floats', 'octseg_mbconv_pool_slots', 'octseg_dwconv_pool_slots', 'octseg_preprocess_resize_s2d',
+    'octseg_fold_average_threshold', 'octseg_contour_largest', 'octseg_dwconv_pool_slots', 'octseg_preprocess_resize_s2d',
 ]
 
 
@@ -82,11 +82,6 @@ def load() -> C.CDLL:
     lib.octseg_dwconv.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int32] * 11 + [
         C.c_void_p, C.c_int32, C.c_void_p]
     lib.octseg_dwconv_pool_slots.argtypes = [C.c_int32, C.c_int32, C.c_int32]
-    lib.octseg_mbconv_pool_slots.argtypes = [C.c_int32, C.c_int32, C.c_int32]
-    lib.octseg_mbconv_expand_dw.argtypes = [C.c_void_p] + [C.c_int32] * 5 + [C.c_void_p] * 3 + [C.c_int32] * 7 + [
-        C.c_void_p, C.c_void_p]
-    lib.octseg_mbconv_smem_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
-    lib.octseg_mbconv_blob_floats.argtypes = [C.c_int32, C.c_int32]
     lib.octseg_se_hidden.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                      C.c_int32, C.c_void_p]
     lib.octseg_se_gate.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
@@ -115,7 +110,7 @@ def load() -> C.CDLL:
     for name in EXPORTS:
         if name not in ('octseg_last_error',):
             getattr(lib, name).restype = C.c_int
-    if lib.octseg_abi_version() != 2:
+    if lib.octseg_abi_version() != 3:
         raise OctsegError('liboctseg.so ABI version mismatch')
     _lib = lib
     return lib
@@ -125,20 +120,6 @@ def check(rc: int, what: str = '') -> None:
     if rc != 0:
         msg = load().octseg_last_error().decode('utf-8', 'replace')
         raise OctsegError(f'{what} failed (code {rc}): {msg}')
-
-
-def mbconv_blob(b_exp, w_dw, b_dw, k: int):
-    """Per-block constants of octseg_mbconv_expand_dw (layout in include/octseg.h): fp32 [ceil(Cmid/64)][2 + k*k][64],
-    rows b_exp/2, b_dw/2, then the k*k depthwise taps/2; w_dw is [k][k][Cmid] (any float dtype: its VALUES are used,
-    so pass bf16-rounded filters to match the unfused kernel)."""
-    import torch
-    cmid = b_exp.numel()
-    ncb = -(-cmid // 64)
-    rows = torch.zeros(2 + k * k, ncb * 64, dtype=torch.float32)
-    rows[0, :cmid] = 0.5 * b_exp.detach().float().cpu()
-    rows[1, :cmid] = 0.5 * b_dw.detach().float().cpu()
-    rows[2:, :cmid] = 0.5 * w_dw.detach().float().cpu().reshape(k * k, cmid)
-    return rows.reshape(2 + k * k, ncb, 64).permute(1, 0, 2).contiguous()
 
 
 def stream_ptr() -> int:

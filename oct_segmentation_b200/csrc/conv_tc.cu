@@ -58,11 +58,6 @@ struct SegK {
   int last_steps;  // K = 16 MMA steps of the LAST chunk that hold real channels (the rest of it is zero padding: skipped)
 };
 
-// 1: one mbarrier arrival per epilogue warp; 0: one per thread (A/B: tools/ab)
-#ifndef OCTSEG_WARP_ARRIVE
-#define OCTSEG_WARP_ARRIVE 1
-#endif
-constexpr int kEpiArrivals = OCTSEG_WARP_ARRIVE ? kEpiWarps : kEpiThreads;
 constexpr int kHeadMaxC = 64;  // channels per pixel a fused 1x1 head can read
 
 struct __align__(64) ConvKParams {
@@ -398,12 +393,12 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
     }
     for (int a = 0; a < p.n_acc; ++a) {
       mbar_init(bar_tfull + 8 * a, 1);
-      mbar_init(bar_tempty + 8 * a, kEpiArrivals);  // one arrival per epilogue WARP (512 per-thread arrivals on one
-                                                 // barrier serialise: ~1000 cycles per tile, the floor of every small tile)
+      mbar_init(bar_tempty + 8 * a, kEpiWarps);  // one arrival per epilogue WARP (512 per-thread arrivals on one
+                                              // barrier serialise: ~1000 cycles per tile, the floor of every small tile)
     }
     mbar_init(bar_bres, 1);
     for (int b = 0; b < kOutBufs; ++b) {
-      mbar_init(bar_sfull + 8 * b, kEpiArrivals / 2);
+      mbar_init(bar_sfull + 8 * b, kEpiWarps / 2);
       mbar_init(bar_sfree + 8 * b, 1);
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -877,7 +872,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
         mbar_wait(bar_tfull + 8 * acc, acc_phase);  // stay within the ring: arrivals must land in this tile's phase
         if (tracer) OCTSEG_STAMP(tev + 1, it);
         __syncwarp();
-        if (!OCTSEG_WARP_ARRIVE || lane == 0) mbar_arrive(bar_tempty + 8 * acc);
+        if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);
         if (tracer) OCTSEG_STAMP(tev + 2, it);
         chunk_ctr += n_tma1;
         if (++acc == p.n_acc) {
@@ -939,7 +934,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
                        : "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncwarp();                                       // every lane's rows written and fenced ...
-        if (!OCTSEG_WARP_ARRIVE || lane == 0) mbar_arrive(bar_sfull + 8 * sbi);    // ... 8 warp arrivals: the store warp issues the TMA store
+        if (lane == 0) mbar_arrive(bar_sfull + 8 * sbi);    // ... 8 warp arrivals: the store warp issues the TMA store
         ++grp_chunks;
         OCTSEG_CSTAMP(4, ckey);
       }
@@ -1015,7 +1010,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
       }
       tc_fence_before();
       __syncwarp();  // every lane's TMEM reads are complete (tcgen05.wait::ld) before the warp's one arrival
-      if (!OCTSEG_WARP_ARRIVE || lane == 0) mbar_arrive(bar_tempty + 8 * acc);
+      if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);
       if (tracer) OCTSEG_STAMP(tev + 2, it);  // accumulator released
       if (++acc == p.n_acc) {
         acc = 0;

@@ -10,7 +10,7 @@
 //     per-thread global address arithmetic); the next tiles' loads fly under the current tile's math;
 //   * a thread owns 4 channels of a 2 x 4 output patch: every shared-memory read uses a compile-time
 //     offset from one per-thread base, each input vector is converted bf16->fp32 once and feeds up to
-//     min(2,K/S) x K taps (vertical + horizontal register reuse); math is packed fp32x2 (FFMA2);
+//     min(2,K/S) x K taps (vertical + horizontal register reuse); math is fp32x2 pairs (FFMA2 for k = 3);
 //   * fp32 filters of the CTA's channel block sit in shared memory, reloaded only when the block changes;
 //   * squeeze-excite sums (of the fp32 activation, before the bf16 rounding) stay in registers across tiles and leave the CTA as one global atomic per
 //     channel when the (image, channel block) changes.
@@ -22,10 +22,115 @@
 #include <cstdint>
 
 #include "common.h"
-#include "dw_core.h"
 #include "ptx_sm100.h"
 
 namespace octseg {
+
+constexpr int kDwR = 2, kDwP = 4;  // output rows x pixels per thread
+
+// Packed FFMA2 or two scalar FFMAs per channel pair.  Measured on B200 (tools/ab/ffma_rate.cu): FFMA2 with three
+// register-pair operands sustains 43-56 FMA lanes/clk/SM, scalar three-register FFMA 73-83, so FFMA2 only pays where the
+// kernel is bound by issue slots (k = 3), not by the FMA pipe (k = 5).
+template <bool PACKED>
+__device__ __forceinline__ float2 dw_fma2(float2 a, float2 b, float2 c) {
+  if (PACKED) return __ffma2_rn(a, b, c);
+  return make_float2(fmaf(a.x, b.x, c.x), fmaf(a.y, b.y, c.y));
+}
+
+// bf16 pair -> fp32 pair on the ALU pipe only (PRMT + LOP3): the compiler would turn `w << 16` into
+// IMAD.U32, which competes with the FFMA2s for the FMA pipe this kernel is bound by
+__device__ __forceinline__ float2 dw_bf16x2_to_f32x2(uint32_t w) {
+  uint32_t lo;
+  asm("prmt.b32 %0, %1, 0, 0x1044;" : "=r"(lo) : "r"(w));
+  return make_float2(__uint_as_float(lo), __uint_as_float(w & 0xffff0000u));
+}
+__device__ __forceinline__ uint32_t dw_cvt_bf16x2(float2 x) {
+  uint32_t d;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(x.y), "f"(x.x));
+  return d;
+}
+__device__ __forceinline__ float dw_tanh(float x) {
+  float y;
+  asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+
+// acc[r][q][0..1] = bias + sum over the K x K taps for the thread's 2 x 4 patch x 4 channels, then the activation.
+//   base : shared-memory address of the thread's window origin (its first row / pixel / channel quad)
+//   w_off: shared-memory address of the thread's 4 channels in the fp32 filter table [K*K][CB] (16-byte aligned)
+// With act == swish the filters and bias are pre-halved by the caller, so the accumulators hold h = x/2 and
+// swish(x) = h*tanh(h) + h costs one FFMA2 + two MUFU per pair.
+template <int K, int S, int CB, int IW, int PIX>
+__device__ __forceinline__ void dw_patch(uint32_t base, uint32_t w_off, const float2 (&bias2)[2], int act,
+                                         float2 (&acc)[kDwR][kDwP][2]) {
+  constexpr int R = kDwR, P = kDwP;
+  constexpr bool PK = K == 3;
+  constexpr int RH = (R - 1) * S + K, RW = (P - 1) * S + K;  // a thread's input window
+#pragma unroll
+  for (int r = 0; r < R; ++r)
+#pragma unroll
+    for (int q = 0; q < P; ++q) {
+      acc[r][q][0] = bias2[0];
+      acc[r][q][1] = bias2[1];
+    }
+#pragma unroll
+  for (int iy = 0; iy < RH; ++iy) {
+    float2 w[R][K][2];
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+      const int ky = iy - r * S;
+      if (ky >= 0 && ky < K) {
+#pragma unroll
+        for (int kx = 0; kx < K; ++kx) {
+          float4 ww;
+          asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
+                       : "=f"(ww.x), "=f"(ww.y), "=f"(ww.z), "=f"(ww.w)
+                       : "r"(w_off + static_cast<uint32_t>((ky * K + kx) * CB * 4)));
+          w[r][kx][0] = make_float2(ww.x, ww.y);
+          w[r][kx][1] = make_float2(ww.z, ww.w);
+        }
+      }
+    }
+#pragma unroll
+    for (int dx = 0; dx < RW; ++dx) {
+      uint32_t r0, r1;
+      asm volatile("ld.shared.v2.b32 {%0, %1}, [%2];"
+                   : "=r"(r0), "=r"(r1)
+                   : "r"(base + static_cast<uint32_t>((iy * IW + dx) * PIX)));
+      const float2 f0 = dw_bf16x2_to_f32x2(r0), f1 = dw_bf16x2_to_f32x2(r1);
+#pragma unroll
+      for (int r = 0; r < R; ++r) {
+        const int ky = iy - r * S;
+        if (ky >= 0 && ky < K) {
+#pragma unroll
+          for (int q = 0; q < P; ++q) {
+            const int kx = dx - q * S;
+            if (kx >= 0 && kx < K) {
+              acc[r][q][0] = dw_fma2<PK>(f0, w[r][kx][0], acc[r][q][0]);
+              acc[r][q][1] = dw_fma2<PK>(f1, w[r][kx][1], acc[r][q][1]);
+            }
+          }
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+#pragma unroll
+    for (int q = 0; q < P; ++q) {
+      float2 y0 = acc[r][q][0], y1 = acc[r][q][1];
+      if (act == OCTSEG_ACT_SWISH) {  // the accumulators hold h = x/2
+        y0 = __ffma2_rn(y0, make_float2(dw_tanh(y0.x), dw_tanh(y0.y)), y0);
+        y1 = __ffma2_rn(y1, make_float2(dw_tanh(y1.x), dw_tanh(y1.y)), y1);
+      } else if (act == OCTSEG_ACT_RELU) {
+        y0 = make_float2(fmaxf(y0.x, 0.f), fmaxf(y0.y, 0.f));
+        y1 = make_float2(fmaxf(y1.x, 0.f), fmaxf(y1.y, 0.f));
+      }
+      acc[r][q][0] = y0;
+      acc[r][q][1] = y1;
+    }
+  }
+}
 
 constexpr int kDwThreads = 256;
 

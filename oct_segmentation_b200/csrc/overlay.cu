@@ -7,7 +7,7 @@
 //   img    = paste(img, colour, fill_lut[k]);  img = paste(img, colour, rim ? rim_alpha : 0)
 // with PIL's paste  out = ((t >> 8) + t) >> 8,  t = dst*(255-a) + src*a + 128.
 //
-// overlay_kernel (the product path): the morphology runs on BIT PLANES -- one 32-bit word = 32 pixels of one
+// overlay_kernel: the morphology runs on BIT PLANES -- one 32-bit word = 32 pixels of one
 // row of one class -- so a dilation / erosion row is a handful of funnel shifts and ORs / ANDs for 32 pixels.
 // One block = 128 x TY output pixels (TY = 32); region = tile + 7 halo rows and one halo word (32 px) per side:
 //   S0  mask words (4 class bytes per pixel, 16-byte loads) -> bit planes M: the 8 lanes of a plane word exchange
@@ -18,21 +18,13 @@
 //       ACT = per 32-pixel word, the classes with any RIM | ANY bit
 //   S4  one warp = 32 pixels of a row: classes absent from the ACT word are skipped warp-uniformly, pixels with a
 //       uniform window take k = 256, only object-boundary pixels compute the binomial sum (5 windows, popcounts).
-// overlay_bytes_kernel is the first, byte-lane version (4 classes = 4 bytes of a word, 32 x 8 tiles), kept as an
-// A/B reference (OCTSEG_OVERLAY_IMPL=bytes).
 #include <cuda_runtime.h>
 #include <cstdint>
-#include <cstdlib>
-#include <cstring>
 
 #include "common.h"
 
 namespace octseg {
 
-constexpr int kOvX = 32, kOvY = 8;
-constexpr int kMW = kOvX + 14, kMH = kOvY + 14;  // mask tile (halo 2 + 2 + 3)
-constexpr int kDW = kOvX + 10, kDH = kOvY + 10;  // dilated tile (halo 2 + 3)
-constexpr int kCW = kOvX + 6, kCH = kOvY + 6;    // closed tile (halo 3)
 constexpr uint32_t kOnes = 0x01010101u;
 
 struct OverlayParams {
@@ -47,125 +39,12 @@ struct OverlayParams {
   uint8_t fill_lut[260]; // alpha of the blurred fill for k = 0..256
 };
 
-// rows of the elliptic structuring elements as bit masks (bit dx+r set = tap present)
-__constant__ uint8_t kEl5[5] = {0x04, 0x1f, 0x1f, 0x1f, 0x04};
-__constant__ uint8_t kEl7[7] = {0x08, 0x3e, 0x7f, 0x7f, 0x7f, 0x3e, 0x08};
-
 __device__ __forceinline__ int reflect101(int v, int n) {  // cv2 BORDER_REFLECT_101 for |overshoot| < n
   if (v < 0) v = -v;
   if (v >= n) v = 2 * (n - 1) - v;
   return v;
 }
 
-__global__ void __launch_bounds__(kOvX* kOvY) overlay_bytes_kernel(const OverlayParams p) {
-  __shared__ uint32_t sm_m[kMH * kMW];
-  __shared__ uint32_t sm_d[kDH * kDW];
-  __shared__ uint32_t sm_c[kCH * kCW];
-  const int n = blockIdx.z;
-  const int x0 = blockIdx.x * kOvX, y0 = blockIdx.y * kOvY;
-  const int tid = threadIdx.y * kOvX + threadIdx.x;
-  const uint32_t* mimg = p.mask + static_cast<size_t>(n) * p.H * p.W;
-
-  // mask tile, bytes normalised to {0,1}; 0 outside the image (dilate's border value)
-  for (int i = tid; i < kMH * kMW; i += kOvX * kOvY) {
-    const int ty = i / kMW, tx = i - ty * kMW;
-    const int y = y0 - 7 + ty, x = x0 - 7 + tx;
-    uint32_t v = 0;
-    if (y >= 0 && y < p.H && x >= 0 && x < p.W) {
-      const uint32_t w = __ldg(mimg + static_cast<size_t>(y) * p.W + x);
-      v = __vminu4(w, kOnes);
-    }
-    sm_m[i] = v;
-  }
-  __syncthreads();
-  // 5x5 dilation; positions outside the image hold all-ones (erode's border value)
-  for (int i = tid; i < kDH * kDW; i += kOvX * kOvY) {
-    const int ty = i / kDW, tx = i - ty * kDW;
-    const int y = y0 - 5 + ty, x = x0 - 5 + tx;
-    uint32_t v = kOnes;
-    if (y >= 0 && y < p.H && x >= 0 && x < p.W) {
-      v = 0;
-#pragma unroll
-      for (int dy = 0; dy < 5; ++dy)
-#pragma unroll
-        for (int dx = 0; dx < 5; ++dx)
-          if ((kEl5[dy] >> dx) & 1) v |= sm_m[(ty + dy) * kMW + tx + dx];
-    }
-    sm_d[i] = v;
-  }
-  __syncthreads();
-  // closed = 5x5 erosion of the dilation (0 outside the image: never read as such, see below)
-  for (int i = tid; i < kCH * kCW; i += kOvX * kOvY) {
-    const int ty = i / kCW, tx = i - ty * kCW;
-    const int y = y0 - 3 + ty, x = x0 - 3 + tx;
-    uint32_t v = 0;
-    if (y >= 0 && y < p.H && x >= 0 && x < p.W) {
-      v = kOnes;
-#pragma unroll
-      for (int dy = 0; dy < 5; ++dy)
-#pragma unroll
-        for (int dx = 0; dx < 5; ++dx)
-          if ((kEl5[dy] >> dx) & 1) v &= sm_d[(ty + dy) * kDW + tx + dx];
-    }
-    sm_c[i] = v;
-  }
-  __syncthreads();
-
-  const int x = x0 + threadIdx.x, y = y0 + threadIdx.y;
-  if (x >= p.W || y >= p.H) return;
-  // 7x7: dilate (outside = 0) and erode (outside = 1) of the closed mask
-  uint32_t dil = 0, ero = kOnes;
-#pragma unroll
-  for (int dy = 0; dy < 7; ++dy) {
-    const int yy = y + dy - 3;
-    const bool yin = yy >= 0 && yy < p.H;
-#pragma unroll
-    for (int dx = 0; dx < 7; ++dx) {
-      if (!((kEl7[dy] >> dx) & 1)) continue;
-      const int xx = x + dx - 3;
-      const bool in = yin && xx >= 0 && xx < p.W;
-      const uint32_t c = sm_c[(threadIdx.y + dy) * kCW + threadIdx.x + dx];
-      dil |= in ? c : 0u;
-      ero &= in ? c : kOnes;
-    }
-  }
-  const uint32_t rim = dil & ~ero;
-  // 5x5 binomial sums (16-bit lanes: classes 0,2 in k02, classes 1,3 in k13), reflected borders
-  uint32_t k02 = 0, k13 = 0;
-#pragma unroll
-  for (int dy = 0; dy < 5; ++dy) {
-    const int ry = reflect101(y + dy - 2, p.H) - y0 + 3;
-    const int wy = dy == 0 || dy == 4 ? 1 : (dy == 2 ? 6 : 4);
-#pragma unroll
-    for (int dx = 0; dx < 5; ++dx) {
-      const int rx = reflect101(x + dx - 2, p.W) - x0 + 3;
-      const int wx = dx == 0 || dx == 4 ? 1 : (dx == 2 ? 6 : 4);
-      const uint32_t c = sm_c[ry * kCW + rx];
-      k02 += static_cast<uint32_t>(wy * wx) * (c & 0x00ff00ffu);
-      k13 += static_cast<uint32_t>(wy * wx) * ((c >> 8) & 0x00ff00ffu);
-    }
-  }
-  const size_t pix = (static_cast<size_t>(n) * p.H + y) * p.W + x;
-  int rgb[3] = {p.img[pix * 3], p.img[pix * 3 + 1], p.img[pix * 3 + 2]};
-  for (int i = 0; i < p.n_order; ++i) {
-    const int c = p.order[i];
-    const uint32_t kk = ((c & 1) ? k13 : k02) >> (16 * (c >> 1)) & 0xffffu;
-    const int a1 = p.fill_lut[kk];
-    const int a2 = ((rim >> (8 * c)) & 1u) ? p.rim_alpha : 0;
-#pragma unroll
-    for (int ch = 0; ch < 3; ++ch) {
-      int t = rgb[ch] * (255 - a1) + p.color[c][ch] * a1 + 128;
-      int v = ((t >> 8) + t) >> 8;
-      t = v * (255 - a2) + p.color[c][ch] * a2 + 128;
-      rgb[ch] = ((t >> 8) + t) >> 8;
-    }
-  }
-  p.out[pix * 3] = static_cast<uint8_t>(rgb[0]);
-  p.out[pix * 3 + 1] = static_cast<uint8_t>(rgb[1]);
-  p.out[pix * 3 + 2] = static_cast<uint8_t>(rgb[2]);
-}
-
-// ---------------------------------------------------------------------------------------------- bit planes
 constexpr int kTileWords = 4;            // 128 output pixels per tile row
 constexpr int kRW = kTileWords + 2;      // region words per row (one halo word per side)
 
@@ -444,12 +323,5 @@ extern "C" int octseg_overlay(const uint8_t* img, const uint8_t* mask, uint8_t* 
   }
   p.rim_alpha = rim_alpha;
   for (int k = 0; k < 257; ++k) p.fill_lut[k] = h_fill_lut[k];
-  static const char* impl = getenv("OCTSEG_OVERLAY_IMPL");  // A/B switch for tools/bench_prepost.py, not an API
-  if (impl && !strcmp(impl, "bytes")) {
-    dim3 grid(cdiv(W, kOvX), cdiv(H, kOvY), N);
-    overlay_bytes_kernel<<<grid, dim3(kOvX, kOvY), 0, static_cast<cudaStream_t>(stream)>>>(p);
-    return check_launch("overlay_bytes_kernel");
-  }
-  if (impl && !strcmp(impl, "ty64")) return launch_overlay<64>(p, static_cast<cudaStream_t>(stream));
   return launch_overlay<32>(p, static_cast<cudaStream_t>(stream));  // 128 x 32 tiles: 0.40 vs 0.47 ms per 32 frames at 1000 x 1000
 }

@@ -93,8 +93,8 @@ class Builder:
         self.op_names: List[str] = []
         self.op_macs: List[Optional[int]] = []   # algorithmic MACs of tensor-core launches, None otherwise
         self.op_bytes: List[int] = []            # algorithmic HBM bytes per op: activations read + written once, + weights
-        self.op_kinds: List[str] = []            # kernel family per op: conv_tc | mbconv | dwconv | se | pack | maxpool
-        self.op_fused_macs = {}                  # op name -> dense expand-conv MACs done inside the fused MBConv kernel
+        self.op_kinds: List[str] = []            # kernel family per op: conv_tc | dwconv | se | pack | maxpool
+        self.op_fused_macs = {}                  # always empty; kept because bench.py reads it (op_fused_macs.get)
         self.macs = 0              # algorithmic MACs of the reference graph (dense count)
         self.tc_launches = 0
         self.launches = 0
@@ -348,11 +348,10 @@ class Builder:
         self._add(name, lambda: op, [x], [out], kind='maxpool')
         return out
 
-    def new_pool(self, C: int, k: int, out_hw: Tuple[int, int], fused: bool) -> torch.Tensor:
-        """Squeeze-excite partial-sum buffer fp32 [N][slots][C] for a depthwise (or fused MBConv) launch of this shape:
-        every slot is written exactly once per launch and octseg_se_hidden adds them in order (no atomics)."""
-        slots = (self.lib.octseg_mbconv_pool_slots(k, out_hw[0], out_hw[1]) if fused
-                 else self.lib.octseg_dwconv_pool_slots(C, out_hw[0], out_hw[1]))
+    def new_pool(self, C: int, out_hw: Tuple[int, int]) -> torch.Tensor:
+        """Squeeze-excite partial-sum buffer fp32 [N][slots][C] for a depthwise launch of this shape: every slot is
+        written exactly once per launch and octseg_se_hidden adds them in order (no atomics)."""
+        slots = self.lib.octseg_dwconv_pool_slots(C, out_hw[0], out_hw[1])
         return torch.zeros(self.N, slots, C, dtype=torch.float32, device=self.device)
 
     def dwconv(self, x: Act, w: torch.Tensor, b: torch.Tensor, *, name: str, k: int, stride: int,
@@ -371,36 +370,6 @@ class Builder:
                                          pool.shape[1] if pool is not None else 0, _lib.stream_ptr()), name)
         self.macs += x.N * out_hw[0] * out_hw[1] * x.C * k * k
         self._add(name, lambda: op, [x], [out], kind='dwconv')
-        return out
-
-    def mbconv_fits(self, cin: int, k: int, stride: int) -> bool:
-        """Can the fused expand + depthwise kernel take this block (shared-memory budget, supported shape)?"""
-        b = self.lib.octseg_mbconv_smem_bytes(cin, k, stride)
-        return 0 < b <= 227 * 1024
-
-    def mbconv_expand_dw(self, x: Act, we: torch.Tensor, be: torch.Tensor, wd: torch.Tensor, bd: torch.Tensor, *,
-                         name: str, k: int, stride: int, pad: Tuple[int, int], out_hw: Tuple[int, int],
-                         pool: Optional[torch.Tensor]) -> Act:
-        """Expand 1x1 (+swish) -> depthwise k x k (+swish) -> SE sums in one launch (csrc/mbconv.cu); the
-        expanded tensor is never written.  we: folded [Cmid, Cin, 1, 1]; wd: folded [Cmid, 1, k, k]."""
-        cmid, cin = we.shape[0], we.shape[1]
-        assert x.C == cin and cin % 16 == 0 and cmid % 8 == 0 and stride == 1
-        out = self.new_act(out_hw[0], out_hw[1], cmid)
-        dev = self.device
-        wek = we.detach().float().reshape(cmid, cin).contiguous().to(torch.bfloat16).to(dev)          # [Cmid][Cin]
-        wdk = wd.detach().float().reshape(cmid, k, k).permute(1, 2, 0).contiguous().to(torch.bfloat16)   # [kh][kw][Cmid], bf16 like octseg_dwconv
-        blob = _lib.mbconv_blob(be, wdk, bd, k).to(dev)
-        self._keep += [wek, blob]
-        lib = self.lib
-
-        def op():   # `pool` (new_pool): write-once per-tile slots, summed by octseg_se_hidden
-            _lib.check(lib.octseg_mbconv_expand_dw(x.t.data_ptr(), x.N, x.H, x.W, cin, x.Cp, wek.data_ptr(), blob.data_ptr(),
-                                                   out.t.data_ptr(), cmid, k, stride, pad[0], pad[1], out_hw[0], out_hw[1],
-                                                   pool.data_ptr() if pool is not None else None, _lib.stream_ptr()), name)
-        exp_macs = x.N * x.H * x.W * cin * cmid
-        self.macs += exp_macs + x.N * out_hw[0] * out_hw[1] * cmid * k * k
-        self._add(name, lambda: op, [x], [out], kind='mbconv', extra_bytes=wek.numel() * 2 + blob.numel() * 4)
-        self.op_fused_macs[name] = exp_macs          # tensor-core MACs executed inside a non-conv_tc kernel
         return out
 
     def se_project(self, x: Act, pool: torch.Tensor, w1, b1, w2, b2, wp: torch.Tensor, bp: torch.Tensor, *,
@@ -423,12 +392,12 @@ class Builder:
         if f > 1:
             wpk, bpk = pack_conv_weights(wp, bp, [x.C], [x.Cp], f, 0, cs)
             spec = [((N, x.H, x.W // f, f * x.Cp, f * x.Cp), False)]
-            geom, packed32 = plan_conv(spec, wpk, out_hw=(x.H, x.W // f), packed_dtype=torch.float32, allow_resident=False)
+            geom, packed32 = plan_conv(spec, wpk, out_hw=(x.H, x.W // f), packed_dtype=torch.float32)
             geom.macs = N * x.H * x.W * cout * C_mid                                # dense count of the real op
             bias_rows = pad_bias(bpk, geom, f * cs)
         else:
             spec = [((N, x.H, x.W, x.C, x.Cp), False)]
-            geom, packed32 = plan_conv(spec, wp, out_hw=(x.H, x.W), packed_dtype=torch.float32, allow_resident=False)
+            geom, packed32 = plan_conv(spec, wp, out_hw=(x.H, x.W), packed_dtype=torch.float32)
             bias_rows = pad_bias(bp, geom, cout)
         rows, Ktot = packed32.shape[1], packed32.shape[2]
         base = packed32[0].contiguous().to(dev)                                    # fp32 [rows][Ktot]

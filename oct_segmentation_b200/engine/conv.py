@@ -19,14 +19,8 @@ import torch
 
 from .. import _lib
 
-import os as _os
-KC64_ALWAYS = _os.environ.get('OCTSEG_KC64', '0') == '1'   # experiment: zero-padded 64-channel chunks for every source
 KC = 64  # K elements per pipeline stage (one 128-byte swizzle atom of bf16)
-WIDE_BOXES = True  # allow shifted-view tap reuse (SegSpec.wide)
-HALO_TILES = True  # allow halo-tile mode (ConvGeom.halo)
 HALO_B_BYTES = 80 * 1024   # resident-weight budget of halo mode (shared memory)
-RES1X1_B_BYTES = 100 * 1024   # ... and of its 1x1 form (three 16 KB A stages remain)
-RESIDENT_1X1 = _os.environ.get('OCTSEG_RES1X1', '0') == '1'   # experiment: resident weights for mid-size 1x1 convs
 
 
 def choose_kc(c_eff: int, taps: int = 9) -> int:
@@ -35,7 +29,7 @@ def choose_kc(c_eff: int, taps: int = 9) -> int:
     (tap, chunk) sub-blocks share one pipeline stage.  A 1x1 conv over 33..48 channels is output-bound: one
     zero-padded 64-channel chunk (one TMA box of 128-byte rows) beats three 16-channel boxes of 32-byte rows
     (measured 48 -> 288 @224^2: 0.23 ms vs 0.34 ms, tools/bench_expand.py)."""
-    if c_eff > 48 or (taps == 1 and c_eff > 32) or KC64_ALWAYS:
+    if c_eff > 48 or (taps == 1 and c_eff > 32):
         return 64
     if c_eff > 32:
         return 16
@@ -172,7 +166,7 @@ def _phase_tap_groups(ph: int, a: int) -> List[int]:
 def plan_conv(srcs: Sequence[Tuple[Tuple[int, int, int, int, int], bool]], weight: torch.Tensor,
               out_hw: Optional[Tuple[int, int]] = None, stride: int = 1, pad: Tuple[int, int] = (0, 0),
               groups: int = 1, transposed: bool = False, out_bf16: bool = True,
-              packed_dtype: torch.dtype = torch.bfloat16, allow_resident: bool = True) -> Tuple[ConvGeom, torch.Tensor]:
+              packed_dtype: torch.dtype = torch.bfloat16) -> Tuple[ConvGeom, torch.Tensor]:
     """Plan one conv.
 
     srcs: [((N, H, W, C, ldc), upsampled)] in concat order; ``upsampled`` sources are at half the
@@ -211,11 +205,11 @@ def plan_conv(srcs: Sequence[Tuple[Tuple[int, int, int, int, int], bool]], weigh
             phases, Hq, Wq = 1, out_H, out_W
         macs = N * out_H * out_W * cout * cin_g * kh * kw
     return _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, tuple(pad), groups, transposed, out_bf16, macs,
-                 packed_dtype, allow_resident and packed_dtype == torch.bfloat16)
+                 packed_dtype)
 
 
 def _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, pad, groups, transposed, out_bf16, macs,
-          packed_dtype=torch.bfloat16, allow_resident=True):
+          packed_dtype=torch.bfloat16):
     cout = w.shape[1] if transposed else w.shape[0]
     cout_w = pad8(cout) if out_bf16 else cout          # channels the kernel writes
     TH, TW = choose_tile(Hq, Wq)
@@ -228,19 +222,6 @@ def _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, pad, groups, transpo
         k_est = sum((2 * 2 if (transposed or up) else (3 * 3 if phases == 4 else w.shape[2] * w.shape[3])) * sC
                     for (_, _, _, sC, _), up in srcs)
         n_tiles_n, BN = choose_bn(max(cout_w, 16), k_est)
-        res1x1 = False
-        if (RESIDENT_1X1 and allow_resident and out_bf16 and len(srcs) == 1 and phases == 1 and not transposed and stride == 1
-                and tuple(w.shape[2:]) == (1, 1) and srcs[0][0][3] >= 128 and cout_w >= 128
-                and Hq * Wq >= 0.75 * (-(-Hq // 16) * 16) * (-(-Wq // 8) * 8)):
-            # mid-size 1x1 conv: every tile re-reads its BN x K weight slice from L2 (stages 4-5 expands of EfficientNet are
-            # bound by that).  Halo-tile mode with a 1x1 "halo" keeps the slice resident in shared memory instead; BN is
-            # the widest whole number of 64-channel chunks whose slice fits.
-            cch = -(-srcs[0][0][3] // 64)
-            bn_max = min(256, RES1X1_B_BYTES // (cch * 128) // 64 * 64)
-            if bn_max >= 128:
-                n_tiles_n = -(-cout_w // bn_max)
-                BN = -(-(-(-cout_w // n_tiles_n)) // 64) * 64
-                res1x1 = True
         cout_per_tile = BN
     rows = n_tiles_n * BN
 
@@ -300,16 +281,14 @@ def _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, pad, groups, transpo
     # (8-pixel rows keep the UMMA 8-row groups at a uniform stride); the channel tile's whole weight
     # slice stays resident in shared memory.  Cuts the L2->smem traffic of such layers ~9x.
     halo = 0
-    if (HALO_TILES and len(segs) == 1 and phases == 1 and not transposed):
+    if len(segs) == 1 and phases == 1 and not transposed:
         sg = segs[0]
         b_bytes = sg.kh * sg.kw * sg.cchunks * BN * sg.kc * 2
         cover = (-(-Hq // 16) * 16) * (-(-Wq // 8) * 8)
         if (sg.mul == 1 and sg.kh * sg.kw >= 4 and sg.kh <= 7 and sg.kw <= 7 and b_bytes <= HALO_B_BYTES
                 and Hq * Wq >= 0.75 * cover):
             halo, TH, TW = 1, 16, 8
-        elif groups == 1 and res1x1 and sg.kc == 64 and b_bytes <= RES1X1_B_BYTES:
-            halo, TH, TW = 1, 16, 8
-    if (TH != 1 and WIDE_BOXES and not halo and phases == 1 and not transposed and BN <= 128
+    if (TH != 1 and not halo and phases == 1 and not transposed and BN <= 128
             and all(sg.kc == 64 and sg.mul == 1 and sg.kw >= 2 and (sg.c_per_tile == 0 or sg.cchunks == 1) for sg in segs)):
         # k x k conv over wide sources with few output channels and no resident-weight (halo) form: L2 -> shared-memory
         # traffic bounds it (every tap re-reads its A tile).  A ROW tile lets the kw taps of a tap row share one box
@@ -325,7 +304,7 @@ def _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, pad, groups, transpo
                 best_tw, best_eff = tw, eff
         if best_eff >= 0.8:
             TH, TW = 1, best_tw
-    if TH == 1 and WIDE_BOXES and not halo:
+    if TH == 1 and not halo:
         # activation-traffic saver for L2-bound shapes: the B stage then holds kw weight tiles
         for sg in segs:
             if (sg.kc == 64 and sg.mul == 1 and sg.kw >= 2 and TW + sg.kw - 1 <= 136 and BN <= 128

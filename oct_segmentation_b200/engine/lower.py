@@ -18,12 +18,6 @@ import torch
 from .builder import Builder, fold_bn
 from .conv import Act
 
-# Fused expand 1x1 + depthwise + SE sums (csrc/mbconv.cu) for the stride-1 MBConv blocks it fits.  It removes the
-# expanded tensor's HBM round trip (stage 2: 1.03 GB per launch instead of 2.9 GB for the pair it replaces) but on
-# B200 the pair is bound by CUDA-core issue / MUFU, not by HBM, and the fused kernel measured 7-50 % SLOWER than
-# the two launches (profiles/mbconv_fused_r2.md), so it is opt-in.  Set of stage input widths to fuse, or () for none.
-FUSE_MBCONV = ()
-
 
 # ----------------------------------------------------------------------------------- encoders
 def lower_resnet(b: Builder, enc, x: torch.Tensor, in_dtype: str, norm) -> List[Act]:
@@ -97,20 +91,12 @@ def lower_efficientnet(b: Builder, enc, x: torch.Tensor, in_dtype: str, norm) ->
         cmid = blk._depthwise_conv.weight.shape[0]
         oh = (y.H + pt + pb - blk.k) // blk.stride + 1
         ow = (y.W + pt + pb - blk.k) // blk.stride + 1
-        fuse = (blk.expand != 1 and cur.C in FUSE_MBCONV and blk.stride == 1 and cur.C % 16 == 0
-                and b.mbconv_fits(cur.C, blk.k, blk.stride))
-        pool = b.new_pool(cmid, blk.k, (oh, ow), fuse)          # fp32 [N][slots][C] partial sums for the SE mean
-        if fuse:
-            # expand 1x1 -> depthwise in one launch: the 6x-wide tensor stays on chip (csrc/mbconv.cu)
+        pool = b.new_pool(cmid, (oh, ow))          # fp32 [N][slots][C] partial sums for the SE mean
+        if blk.expand != 1:
             we, be = fold_bn(blk._expand_conv.weight, blk._bn0)
-            y = b.mbconv_expand_dw(y, we, be, wd, bd, name=nm + '._depthwise_conv', k=blk.k, stride=blk.stride,
-                                   pad=(pt, pt), out_hw=(oh, ow), pool=pool)
-        else:
-            if blk.expand != 1:
-                we, be = fold_bn(blk._expand_conv.weight, blk._bn0)
-                y = b.conv([(y, False)], we, be, name=nm + '._expand_conv', act='swish')
-            y = b.dwconv(y, wd, bd, name=nm + '._depthwise_conv', k=blk.k, stride=blk.stride, pad=(pt, pt),
-                         out_hw=(oh, ow), act='swish', pool=pool)
+            y = b.conv([(y, False)], we, be, name=nm + '._expand_conv', act='swish')
+        y = b.dwconv(y, wd, bd, name=nm + '._depthwise_conv', k=blk.k, stride=blk.stride, pad=(pt, pt),
+                     out_hw=(oh, ow), act='swish', pool=pool)
         wp, bp = fold_bn(blk._project_conv.weight, blk._bn2)
         skip = inp if (blk.stride == 1 and blk.cin == blk.cout) else None
         cur = b.se_project(y, pool, blk._se_reduce.weight, blk._se_reduce.bias, blk._se_expand.weight,
@@ -159,11 +145,6 @@ def lower_unetpp_decoder(b: Builder, dec, feats: List[Act]) -> Act:
     return _unet_block(b, dec.blocks[key], dense[f'x_0_{depth - 1}'], [], 'decoder.blocks.' + key)
 
 
-# LinkNet ends in conv1x1+BN+ReLU (16 -> 32 channels at full resolution) followed by a 1x1 segmentation head: fused, the
-# 32-channel full-resolution tensor (the largest activation of the network) is never written or read back.
-FUSE_LINKNET_HEAD = True
-
-
 def lower_linknet_decoder(b: Builder, dec, feats: List[Act], head=None) -> Optional[Act]:
     """head = (segmentation_head, out tensor, out_mode): fuse the 1x1 head into the last block's final conv; returns
     None then (there is no decoder output tensor any more)."""
@@ -203,8 +184,9 @@ def lower_decoder_and_head(b: Builder, model, feats: List[Act], out: torch.Tenso
     """Decoder + segmentation head into ``out``.  Returns the decoder's output activation, or None when the head was
     fused into the decoder's last conv (LinkNet: its 1x1 head rides in that conv's epilogue)."""
     head = model.segmentation_head
-    if (model.decoder.kind == 'linknet' and FUSE_LINKNET_HEAD and tuple(head[0].kernel_size) == (1, 1)
-            and head[0].out_channels <= 4):
+    # LinkNet ends in conv1x1+BN+ReLU (16 -> 32 channels at full resolution) followed by a 1x1 segmentation head: fused,
+    # the 32-channel full-resolution tensor (the largest activation of the network) is never written or read back.
+    if model.decoder.kind == 'linknet' and tuple(head[0].kernel_size) == (1, 1) and head[0].out_channels <= 4:
         return lower_linknet_decoder(b, model.decoder, feats, head=(head, out, out_mode))
     y = DECODER_LOWERING[model.decoder.kind](b, model.decoder, feats)
     lower_head(b, head, y, out, out_mode)

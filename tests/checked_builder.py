@@ -65,19 +65,6 @@ class CheckedBuilder(Builder):
         self.checks.append((k['name'], ref_fn, lambda: _nchw(out)))
         return out
 
-    def mbconv_expand_dw(self, x, we, be, wd, bd, **k):
-        out = super().mbconv_expand_dw(x, we, be, wd, bd, **k)
-        pool = k['pool']
-
-        def ref_fn():
-            kk = dict(k)
-            kk['pool'] = torch.zeros_like(pool)
-            r = _nchw(self.ref.mbconv_expand_dw(x, we, be, wd, bd, **kk))
-            self._last_pool_err = _rel(pool.sum(1), kk['pool'].sum(1))
-            return r
-        self.checks.append((k['name'], ref_fn, lambda: _nchw(out)))
-        return out
-
     def se_project(self, x, pool, w1, b1, w2, b2, wp, bp, **k):
         out = super().se_project(x, pool, w1, b1, w2, b2, wp, bp, **k)
         self._pools[k['name'] + '.se'] = pool

@@ -73,16 +73,8 @@ class CpuBuilder:
         pool[:, 0].copy_(y.sum(dim=(2, 3)))
         return _act(y)
 
-    def new_pool(self, C, k, out_hw, fused):
+    def new_pool(self, C, out_hw):
         return torch.zeros(self.N, 1, C, device=self.device)
-
-    def mbconv_fits(self, cin, k, stride):
-        return stride == 1 and cin % 16 == 0 and cin <= 160
-
-    def mbconv_expand_dw(self, x, we, be, wd, bd, *, name, k, stride, pad, out_hw, pool):
-        """The fused kernel's contract = the two separate ops (the Bf16 subclass rounds the expanded tensor)."""
-        y = self.conv([(x, False)], we, be, name=name + '.expand', act='swish')
-        return self.dwconv(y, wd, bd, name=name, k=k, stride=stride, pad=pad, out_hw=out_hw, act='swish', pool=pool)
 
     def se_project(self, x, pool, w1, b1, w2, b2, wp, bp, *, name, res):
         xin = _nchw(x)

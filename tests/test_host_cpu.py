@@ -24,7 +24,7 @@ def test_library_exports_every_declared_symbol():
     lib = ctypes.CDLL(_lib.LIB_PATH)
     for name in declared:
         assert hasattr(lib, name), name
-    assert _lib.load().octseg_abi_version() == 2
+    assert _lib.load().octseg_abi_version() == 3
 
 
 def test_conv_plan_rejects_bad_arguments_without_a_gpu():

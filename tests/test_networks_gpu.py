@@ -60,21 +60,6 @@ def test_every_launch_matches_torch_in_situ(key):
     assert not bad, f'{key}: launches off by more than 1e-2: {bad[:8]}'
 
 
-def test_every_launch_matches_torch_in_situ_with_fused_mbconv(monkeypatch):
-    """FC_LC lowered with the opt-in fused expand + depthwise kernel (engine/lower.py FUSE_MBCONV) for every stage
-    width it supports: each fused launch is checked against the two torch ops it replaces, on its own inputs."""
-    from oct_segmentation_b200.engine import lower
-    monkeypatch.setattr(lower, 'FUSE_MBCONV', (32, 48, 80, 160, 224))
-    ref, ours = build_pair('FC_LC')
-    x = torch.from_numpy(frames_bgr(2, 192)).cuda()
-    net = CompiledNet(ours.model, 2, 192, 192, x.device, 'u8', 'f32_nchw', use_graph=False, builder_cls=CheckedBuilder)
-    assert 'mbconv' in net.builder.op_kinds
-    net.x_nhwc.copy_(x)
-    errs = net.builder.run_checked()
-    bad = [(n, e) for n, e in errs if not e <= 1e-2]
-    assert not bad, f'fused MBConv launches off by more than 1e-2: {bad[:8]}'
-
-
 @pytest.mark.parametrize('key,H,W,N', [('LM', 96, 160, 3), ('VV', 224, 160, 3), ('FC_LC', 160, 224, 1)])
 def test_every_launch_matches_torch_in_situ_non_square(key, H, W, N):
     """Same per-launch check on non-square inputs and odd batch sizes: feature maps such as 7x5, 14x10, 28x20

@@ -1,4 +1,4 @@
-// Microbenchmark: FP32 FMA issue rates on sm_100a by operand form, to bound the depthwise kernel (csrc/dw_core.h).
+// Microbenchmark: FP32 FMA issue rates on sm_100a by operand form, to bound the depthwise kernel (csrc/dwconv.cu).
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o tools/ab/ffma_rate tools/ab/ffma_rate.cu && tools/ab/ffma_rate
 // One CTA of 512 threads per SM (4 warps per scheduler); every variant runs ITERS x 16 independent FMA(2)s per thread
 // and reports FMA lanes per clock per SM from clock64().

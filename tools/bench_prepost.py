@@ -75,7 +75,7 @@ def main():
     b = N * HO * HO * (3 + 4 + 3)
     for what, mm in (('OCT-shaped masks', [shaped] * sets), ('noise masks (worst case)', masks)):
         ms = timeit([lambda i=i: prepost.overlay(big[i], mm[i], [0, 1, 2, 3], overs[i]) for i in range(sets)])
-        print(json.dumps(dict(kernel='overlay', masks=what, impl=os.environ.get('OCTSEG_OVERLAY_IMPL', 'default'), Ho=HO, frames=N,
+        print(json.dumps(dict(kernel='overlay', masks=what, Ho=HO, frames=N,
                               ms=round(ms, 4), GBps=round(b / ms / 1e6, 1), frac_of_hbm=round(b / ms / 1e6 / peak, 3))), flush=True)
     for what, mm in (('OCT-shaped masks', shaped), ('noise masks (worst case)', masks[0])):
         ms = timeit([lambda: prepost.contour_largest(mm)], reps=3)

@@ -40,8 +40,8 @@ def main():
         ms = times.get(name)
         if ms is None:
             continue
-        macs = macs or b.op_fused_macs.get(name, 0)
-        tf = 2 * macs * NB / ms / 1e9 if macs else 0.0
+        macs = macs or 0
+        tf =2 * macs * NB / ms / 1e9 if macs else 0.0
         gbs = byt * NB / ms / 1e6
         ideal = max(2 * macs * NB / 1e9 / peak_tf, byt * NB / 1e6 / peak_gbs)
         rows.append((ms - ideal, name, kind, ms, tf, gbs, ideal))

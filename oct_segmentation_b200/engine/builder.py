@@ -17,7 +17,8 @@ from typing import Callable, List, Optional, Sequence, Tuple
 import torch
 
 from .. import _lib
-from .conv import Act, ConvPlan, d2s_weights, pack_conv_weights, pad8, pad_bias, pixel_pack_factor, plan_conv
+from .conv import (Act, ConvGeom, ConvPlan, d2s_weights, dense_macs, pad8, pad_bias, pixel_pack_factor, plan_conv,
+                   plan_pixel_packed)
 
 
 def fold_bn(w: torch.Tensor, bn: Optional[torch.nn.BatchNorm2d], conv_bias: Optional[torch.Tensor] = None,
@@ -53,10 +54,13 @@ def stem_s2d_weights(w: torch.Tensor, k: int, pad: Tuple[int, int]) -> Tuple[tor
 
 
 class _Op:
-    __slots__ = ('name', 'make', 'reads', 'writes', 'tc_macs')
+    """One recorded op.  kind: kernel family (conv_tc | dwconv | se | pack | maxpool); macs: algorithmic MACs of a
+    tensor-core launch, None otherwise; nbytes: algorithmic HBM bytes (activations read + written once, + weights)."""
+    __slots__ = ('name', 'kind', 'make', 'reads', 'writes', 'macs', 'nbytes')
 
-    def __init__(self, name, make, reads, writes, tc_macs):
-        self.name, self.make, self.reads, self.writes, self.tc_macs = name, make, reads, writes, tc_macs
+    def __init__(self, name, kind, make, reads, writes, macs, nbytes):
+        self.name, self.kind, self.make, self.reads, self.writes = name, kind, make, reads, writes
+        self.macs, self.nbytes = macs, nbytes
 
 
 def plan_arena(items: Sequence[Tuple[int, int, int]], align: int = 256) -> Tuple[List[int], int]:
@@ -89,14 +93,9 @@ class Builder:
         self.device = torch.device(device)
         self.N = N
         self.reuse = reuse           # False: every activation keeps its own bytes (in-situ checks read dead inputs)
-        self.ops: List[Callable[[], None]] = []
-        self.op_names: List[str] = []
-        self.op_macs: List[Optional[int]] = []   # algorithmic MACs of tensor-core launches, None otherwise
-        self.op_bytes: List[int] = []            # algorithmic HBM bytes per op: activations read + written once, + weights
-        self.op_kinds: List[str] = []            # kernel family per op: conv_tc | dwconv | se | pack | maxpool
+        self.ops: List[Callable[[], None]] = []   # one launch function per record, created by finalize()
         self.op_fused_macs = {}                  # always empty; kept because bench.py reads it (op_fused_macs.get)
         self.macs = 0              # algorithmic MACs of the reference graph (dense count)
-        self.tc_launches = 0
         self.launches = 0
         self.act_bytes = 0         # sum of all activation buffers (what a no-reuse allocation would take)
         self.arena_bytes = 0       # bytes actually allocated for them
@@ -105,6 +104,23 @@ class Builder:
         self._pinned: List[Act] = []
         self._keep: List[object] = []
         self._final = False
+
+    # per-op views of the op records (see _Op)
+    @property
+    def op_names(self) -> Tuple[str, ...]:
+        return tuple(op.name for op in self._records)
+
+    @property
+    def op_kinds(self) -> Tuple[str, ...]:
+        return tuple(op.kind for op in self._records)
+
+    @property
+    def op_macs(self) -> Tuple[Optional[int], ...]:
+        return tuple(op.macs for op in self._records)
+
+    @property
+    def op_bytes(self) -> Tuple[int, ...]:
+        return tuple(op.nbytes for op in self._records)
 
     # ------------------------------------------------------------------ buffers
     def new_act(self, H: int, W: int, C: int) -> Act:
@@ -124,15 +140,13 @@ class Builder:
         """Keep these buffers intact until the end of the network (feature taps read by diagnostics)."""
         self._pinned += list(acts)
 
-    def _add(self, name: str, make: Callable[[], Callable[[], None]], reads: Sequence[Act] = (),
-             writes: Sequence[Act] = (), tc_macs: Optional[int] = None, launches: int = 1, extra_bytes: int = 0,
-             kind: str = '') -> None:
+    def _add(self, name: str, make: Callable[[], Callable[[], None]], reads: Sequence[Optional[Act]] = (),
+             writes: Sequence[Act] = (), *, kind: str, macs: Optional[int] = None, launches: int = 1,
+             extra_bytes: int = 0) -> None:
         assert not self._final, 'builder already finalized'
-        self.op_kinds.append(kind or ('conv_tc' if tc_macs is not None else 'other'))
-        self._records.append(_Op(name, make, [a for a in reads if a is not None], list(writes), tc_macs))
-        self.op_names.append(name)
-        self.op_macs.append(tc_macs)
-        self.op_bytes.append(sum(a.nbytes for a in list(reads) + list(writes) if a is not None) + int(extra_bytes))
+        reads, writes = [a for a in reads if a is not None], list(writes)
+        nbytes = sum(a.nbytes for a in reads + writes) + int(extra_bytes)
+        self._records.append(_Op(name, kind, make, reads, writes, macs, nbytes))
         self.launches += launches
 
     def plan_buffers(self) -> Tuple[List[Act], List[int], int]:
@@ -171,7 +185,8 @@ class Builder:
             a.t = self._arena[off:off + a.nbytes].view(a.dtype).view(a.shape)
         self._final = True
         self.ops = [op.make() for op in self._records]
-        self._records = []
+        for op in self._records:
+            op.make = None           # the plans hold what they launch; free the host-side packed weights
 
     def run(self) -> None:
         self.finalize()
@@ -179,15 +194,38 @@ class Builder:
             op()
 
     # ------------------------------------------------------------------ tensor-core conv
-    def _add_conv(self, name: str, geom, make_plan: Callable[[], ConvPlan], reads, writes, extra_bytes: int = 0) -> None:
+    def _add_conv(self, name: str, srcs: List[Act], geom: ConvGeom, packed: torch.Tensor | Act,
+                  bias_rows: torch.Tensor, macs: int,
+                  out_hw: Tuple[int, int], cout: int, f: int = 0, *, act: str, res: Optional[Act] = None,
+                  res_mode: str = 'none', out_mode: str = 'bf16_nhwc', out_tensor: Optional[torch.Tensor] = None,
+                  **plan_kw) -> Optional[Act]:
+        """Records one planned tensor-core conv: allocates its bf16 NHWC output (or checks the NCHW `out_tensor`),
+        counts its MACs and bytes and creates its ConvPlan at finalize().  f > 1: sources, output and residual are
+        seen through their f-pixel packed view.  `packed` is the weight tensor, or the arena buffer of per-image
+        weights (se_project); `plan_kw` are the form's extra ConvPlan arguments."""
+        out, out_bytes = None, 0
+        if out_mode == 'bf16_nhwc':
+            out = self.new_act(out_hw[0], out_hw[1], cout)
+        else:
+            planes = plan_kw['head'][0].shape[0] if 'head' in plan_kw else cout
+            assert out_tensor is not None and tuple(out_tensor.shape) == (self.N, planes) + tuple(out_hw) and res is None
+            out_bytes = out_tensor.numel() * out_tensor.element_size()
+        arena_w = packed if isinstance(packed, Act) else None
+
+        def view(t):        # the pixel-packed view of an NHWC tensor (same memory, f pixels per row)
+            return t.view(t.shape[0], t.shape[1], t.shape[2] // f, f * t.shape[3]) if f > 1 else t
+
         def make():
-            plan = make_plan()
+            plan = ConvPlan(geom, arena_w.t if arena_w is not None else packed, bias_rows, [view(a.t) for a in srcs],
+                            view(out.t) if out is not None else out_tensor, out_mode=out_mode, act=act,
+                            res=view(res.t) if res is not None else None, res_mode=res_mode, name=name, **plan_kw)
             self._keep.append(plan)
             return plan.run
-        self.macs += geom.macs
-        self.tc_launches += 1
+        self.macs += macs
         wbytes = geom.phases * geom.n_tiles_n * geom.BN * geom.Ktot * 2
-        self._add(name, make, reads, writes, tc_macs=geom.macs, extra_bytes=extra_bytes + wbytes)
+        self._add(name, make, srcs + [res, arena_w], [out] if out is not None else [], kind='conv_tc', macs=macs,
+                  extra_bytes=out_bytes + wbytes)
+        return out
 
     def conv(self, srcs: Sequence[Tuple[Act, bool]], w: torch.Tensor, b: Optional[torch.Tensor], *, name: str,
              stride: int = 1, pad: Tuple[int, int] = (0, 0), groups: int = 1, transposed: bool = False,
@@ -200,99 +238,60 @@ class Builder:
         head's logits / masks and the conv's own output is never stored."""
         cout = w.shape[1] if transposed else w.shape[0]
         bf16_out = out_mode == 'bf16_nhwc'
-        reads = [a for a, _ in srcs] + [res]
-        head_t, n_planes = None, cout
-        if head is not None:
-            hw = head[0].detach().float().cpu().reshape(head[0].shape[0], -1)
-            assert not bf16_out and res is None and not transposed and hw.shape[1] == cout and cout % 16 == 0 and hw.shape[0] <= 4
-            hb = head[1].detach().float().cpu() if head[1] is not None else torch.zeros(hw.shape[0])
-            cb = b.detach().float().cpu() if b is not None else torch.zeros(cout)
-            assert cout <= 64, 'a fused head reads at most 64 channels per pixel'
-            head_t, n_planes = (hw, hb, cb), hw.shape[0]
-        # narrow stride-1 convs: pack f adjacent pixels into one GEMM row (same memory, wider view)
-        f = 0
-        if (not transposed and groups == 1 and stride == 1 and not any(up for _, up in srcs) and out_hw is None
-                and pad[0] == (w.shape[2] - 1) // 2 and pad[1] == (w.shape[3] - 1) // 2):
-            f = pixel_pack_factor([a.Cp for a, _ in srcs], srcs[0][0].W, w.shape[3], pad8(cout) if bf16_out else cout)
-            if head_t is not None and f > 4:
-                f = 4                                         # the fused-head epilogue packs at most 4 pixels per row
-        if f:
-            a0 = srcs[0][0]
-            cout_store = pad8(cout) if bf16_out else cout
-            wp, bp = pack_conv_weights(w, b, [a.C for a, _ in srcs], [a.Cp for a, _ in srcs], f, pad[1], cout_store)
-            spec = [((a.N, a.H, a.W // f, f * a.Cp, f * a.Cp), False) for a, _ in srcs]
-            geom, packed = plan_conv(spec, wp, stride=1, pad=(pad[0], 1 if w.shape[3] > 1 else 0), out_bf16=bf16_out)
-            geom.macs = a0.N * a0.H * a0.W * cout * w.shape[1] * w.shape[2] * w.shape[3]     # dense count of the real op
-            bias_rows = pad_bias(bp, geom, f * cout_store)
-            out_act = None
-            if bf16_out:
-                out_act = self.new_act(a0.H, a0.W, cout)
-            else:
-                assert out_tensor is not None and tuple(out_tensor.shape) == (self.N, n_planes, a0.H, a0.W) and res is None
-            if head_t is not None:
-                geom.macs += a0.N * a0.H * a0.W * cout * n_planes
-
-            def make_plan():
-                views = [a.t.view(a.N, a.H, a.W // f, f * a.Cp) for a, _ in srcs]
-                if bf16_out:
-                    out_t = out_act.t.view(a0.N, a0.H, a0.W // f, f * cout_store)
-                    res_t = res.t.view(a0.N, a0.H, a0.W // f, f * cout_store) if res is not None else None
-                    return ConvPlan(geom, packed, bias_rows, views, out_t, out_mode=out_mode, act=act, res=res_t,
-                                    res_mode=res_mode, name=name)
-                return ConvPlan(geom, packed, bias_rows, views, out_tensor, out_mode=out_mode, act=act, name=name,
-                                out_pack=f, out_ldc=n_planes, head=head_t)
-            self._add_conv(name, geom, make_plan, reads, [out_act] if out_act is not None else [],
-                           extra_bytes=0 if bf16_out else out_tensor.numel() * out_tensor.element_size())
-            return out_act
+        cout_store = pad8(cout) if bf16_out else cout        # channels per output pixel in memory
+        acts, ups = [a for a, _ in srcs], [up for _, up in srcs]
+        a0 = acts[0]
 
         # narrow decoder conv over cat([up(x), skips...]): the half-resolution tile grid of the fused form
         # reads the full-resolution skips through stride-2 boxes, 9 per tile and phase, and is bound by
         # that activation feed.  Split it: depth-to-space conv of the upsampled part (no bias/act), then a
         # plain 3x3 conv of the skips (wide boxes: 3x less feed) that adds the first part before the
         # activation.  Costs one extra bf16 round trip of the (narrow) output.
-        if (bf16_out and not transposed and len(srcs) > 1 and srcs[0][1] and not any(up for _, up in srcs[1:])
-                and groups == 1 and res is None and cout <= 64 and srcs[1][0].W >= 112):
-            cup = srcs[0][0].C
-            part = self.conv([srcs[0]], w[:, :cup], None, name=name + '.up', pad=(1, 1), act='none')
-            return self.conv(list(srcs[1:]), w[:, cup:], b, name=name, pad=(1, 1), act=act, res=part,
+        if (bf16_out and not transposed and len(srcs) > 1 and ups[0] and not any(ups[1:]) and groups == 1
+                and res is None and cout <= 64 and acts[1].W >= 112):
+            part = self.conv([srcs[0]], w[:, :a0.C], None, name=name + '.up', pad=(1, 1), act='none')
+            return self.conv(list(srcs[1:]), w[:, a0.C:], b, name=name, pad=(1, 1), act=act, res=part,
                              res_mode='before_act')
 
-        # single-source upsample+conv / ConvTranspose with few output channels: one depth-to-space conv
-        # on the half-resolution grid (N = 4*Cout) instead of four N = Cout phase problems
-        if (bf16_out and len(srcs) == 1 and (transposed or srcs[0][1]) and res is None and 4 * pad8(cout) <= 256
+        f, plan_kw = 0, {}
+        if (not transposed and groups == 1 and stride == 1 and not any(ups) and out_hw is None
+                and pad[0] == (w.shape[2] - 1) // 2 and pad[1] == (w.shape[3] - 1) // 2):
+            # the fused-head epilogue packs at most 4 pixels per row
+            f = pixel_pack_factor([a.Cp for a in acts], a0.W, w.shape[3], cout_store, 8 if head is None else 4)
+        if f:
+            # narrow stride-1 convs: pack f adjacent pixels into one GEMM row (same memory, wider view)
+            geom, packed, bias_rows = plan_pixel_packed(acts, w, b, f, pad, cout_store, out_bf16=bf16_out)
+            out_hw = (a0.H, a0.W)
+            if not bf16_out:
+                plan_kw['out_pack'] = f
+        elif (bf16_out and len(srcs) == 1 and (transposed or ups[0]) and res is None and 4 * cout_store <= 256
                 and groups == 1):
-            a0 = srcs[0][0]
-            cs = pad8(cout)
-            wp, bp = d2s_weights(w, b, transposed, cs)
+            # single-source upsample+conv / ConvTranspose with few output channels: one depth-to-space conv
+            # on the half-resolution grid (N = 4*Cout) instead of four N = Cout phase problems
+            wp, bp = d2s_weights(w, b, transposed, cout_store)
             geom, packed = plan_conv([((a0.N, a0.H, a0.W, a0.C, a0.Cp), False)], wp, pad=(1, 1))
-            cin = w.shape[0] if transposed else w.shape[1]
-            geom.macs = a0.N * a0.H * a0.W * cin * cout * (16 if transposed else 36)   # dense count of the real op
-            out_act = self.new_act(2 * a0.H, 2 * a0.W, cout)
-            bias_rows = pad_bias(bp, geom, 4 * cs)
-            self._add_conv(name, geom, lambda: ConvPlan(geom, packed, bias_rows, [a0.t], out_act.t, act=act, name=name,
-                                                        out_ldc=out_act.Cp, d2s=cs), reads, [out_act])
-            return out_act
-
-        spec = [((a.N, a.H, a.W, a.C, a.Cp), up) for a, up in srcs]
-        geom, packed = plan_conv(spec, w, out_hw=out_hw, stride=stride, pad=pad, groups=groups,
-                                 transposed=transposed, out_bf16=bf16_out)
-        bias_rows = pad_bias(b, geom, cout, groups)
-        out_act = None
-        if bf16_out:
-            out_act = self.new_act(geom.out_H, geom.out_W, cout)
+            bias_rows = pad_bias(bp, geom, 4 * cout_store)
+            out_hw = (2 * a0.H, 2 * a0.W)
+            plan_kw['d2s'] = cout_store
         else:
-            assert out_tensor is not None and tuple(out_tensor.shape) == (self.N, n_planes, geom.out_H, geom.out_W)
-        if head_t is not None:
-            assert geom.n_tiles_n == 1, 'a fused head needs all of a pixel\'s channels in one tile'
-            geom.macs += self.N * geom.out_H * geom.out_W * cout * n_planes
+            geom, packed = plan_conv([((a.N, a.H, a.W, a.C, a.Cp), up) for a, up in srcs], w, out_hw=out_hw,
+                                     stride=stride, pad=pad, groups=groups, transposed=transposed, out_bf16=bf16_out)
+            bias_rows = pad_bias(b, geom, cout, groups)
+            out_hw = (geom.out_H, geom.out_W)
+        macs = dense_macs(w, self.N, out_hw, transposed)
 
-        def make_plan():
-            return ConvPlan(geom, packed, bias_rows, [a.t for a, _ in srcs], out_act.t if bf16_out else out_tensor,
-                            out_mode=out_mode, act=act, res=res.t if res is not None else None, res_mode=res_mode,
-                            name=name, out_ldc=None if head_t is None else n_planes, head=head_t)
-        self._add_conv(name, geom, make_plan, reads, [out_act] if out_act is not None else [],
-                       extra_bytes=0 if bf16_out else out_tensor.numel() * out_tensor.element_size())
-        return out_act
+        if head is not None:
+            hw = head[0].detach().float().cpu().reshape(head[0].shape[0], -1)
+            assert (not bf16_out and res is None and not transposed and hw.shape[1] == cout and cout % 16 == 0
+                    and hw.shape[0] <= 4)
+            assert cout <= 64, 'a fused head reads at most 64 channels per pixel'
+            assert geom.n_tiles_n == 1, 'a fused head needs all of a pixel\'s channels in one tile'
+            hb = head[1].detach().float().cpu() if head[1] is not None else torch.zeros(hw.shape[0])
+            cb = b.detach().float().cpu() if b is not None else torch.zeros(cout)
+            plan_kw['head'] = (hw, hb, cb)
+            macs += dense_macs(hw, self.N, out_hw)
+        return self._add_conv(name, acts, geom, packed, bias_rows, macs, out_hw, cout, f, act=act, res=res,
+                              res_mode=res_mode, out_mode=out_mode, out_tensor=out_tensor, **plan_kw)
 
     # ------------------------------------------------------------------ CUDA-core kernels
     def stem(self, x: torch.Tensor, in_dtype: str, w: torch.Tensor, b: torch.Tensor, *, name: str, k: int,
@@ -330,12 +329,9 @@ class Builder:
             self._add(name + '.pack', lambda: pack_op, [], [x2], kind='pack', extra_bytes=N * H * W * 3 * (1 if in_dtype == 'u8' else 4))
         w2, q0 = stem_s2d_weights(w, k, pad)
         assert q0[0] <= 0 and q0[1] <= 0
-        out = self.conv([(x2, False)], w2, b, name=name, pad=(-q0[0], -q0[1]), out_hw=out_hw, act=act)
-        real = N * out_hw[0] * out_hw[1] * cout * 3 * k * k        # algorithmic MACs: the dense count of the real op
-        self.macs += real - self.op_macs[-1]
-        self.op_macs[-1] = real
-        self._records[-1].tc_macs = real
-        return out
+        geom, packed = plan_conv([((x2.N, x2.H, x2.W, x2.C, x2.Cp), False)], w2, out_hw=out_hw, pad=(-q0[0], -q0[1]))
+        return self._add_conv(name, [x2], geom, packed, pad_bias(b, geom, cout), dense_macs(w, N, out_hw), out_hw, cout,
+                              act=act)
 
     def maxpool(self, x: Act, *, name: str) -> Act:
         Ho, Wo = (x.H + 2 - 3) // 2 + 1, (x.W + 2 - 3) // 2 + 1
@@ -390,19 +386,13 @@ class Builder:
         # output rows are 128 bytes and K is a whole 64-channel chunk (same memory, wider view; block-diagonal weights)
         f = 2 if (cs <= 32 and x.Cp <= 64 and x.C == x.Cp and x.W % 2 == 0 and (res is None or res.Cp == cs)) else 1
         if f > 1:
-            wpk, bpk = pack_conv_weights(wp, bp, [x.C], [x.Cp], f, 0, cs)
-            spec = [((N, x.H, x.W // f, f * x.Cp, f * x.Cp), False)]
-            geom, packed32 = plan_conv(spec, wpk, out_hw=(x.H, x.W // f), packed_dtype=torch.float32)
-            geom.macs = N * x.H * x.W * cout * C_mid                                # dense count of the real op
-            bias_rows = pad_bias(bpk, geom, f * cs)
+            geom, packed32, bias_rows = plan_pixel_packed([x], wp, bp, f, (0, 0), cs, packed_dtype=torch.float32)
         else:
-            spec = [((N, x.H, x.W, x.C, x.Cp), False)]
-            geom, packed32 = plan_conv(spec, wp, out_hw=(x.H, x.W), packed_dtype=torch.float32)
+            geom, packed32 = plan_conv([((N, x.H, x.W, x.C, x.Cp), False)], wp, packed_dtype=torch.float32)
             bias_rows = pad_bias(bp, geom, cout)
         rows, Ktot = packed32.shape[1], packed32.shape[2]
         base = packed32[0].contiguous().to(dev)                                    # fp32 [rows][Ktot]
         wn = self.new_scratch((N, rows, Ktot), torch.bfloat16)                     # per-image weights: dead after the conv
-        out = self.new_act(x.H, x.W, cout)
         self._keep += [w1d, b1d, w2d, b2d, hidden, gate, base]
         lib, inv_hw = self.lib, 1.0 / float(x.H * x.W)
 
@@ -416,11 +406,6 @@ class Builder:
                                                    f * C_mid, C_mid, st), name + '.se_scale_weights')
         self.macs += N * 2 * C_mid * cr
         self._add(name + '.se', lambda: gate_op, [], [wn], launches=3 + int(pool.shape[1] > 1), kind='se')
-        def make_plan():
-            def pk(t):      # the pixel-packed view of an NHWC tensor
-                return t.view(t.shape[0], t.shape[1], t.shape[2] // f, f * t.shape[3]) if f > 1 else t
-            return ConvPlan(geom, wn.t, bias_rows, [pk(x.t)], pk(out.t), act='none',
-                            res=pk(res.t) if res is not None else None,
-                            res_mode='before_act' if res is not None else 'none', per_image_weights=True, name=name)
-        self._add_conv(name, geom, make_plan, [x, res, wn], [out])
-        return out
+        return self._add_conv(name, [x], geom, wn, bias_rows, dense_macs(wp, N, (x.H, x.W)), (x.H, x.W), cout, f,
+                              act='none', res=res, res_mode='before_act' if res is not None else 'none',
+                              per_image_weights=True)

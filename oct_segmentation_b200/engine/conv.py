@@ -123,8 +123,15 @@ class ConvGeom:
     Ktot: int
     out_H: int
     out_W: int
-    macs: int = 0        # algorithmic MACs of the reference op (dense count, for rooflines)
     halo: int = 0        # 1: 16x8 tiles, one halo-box A load per channel chunk, weights resident in smem
+
+
+def dense_macs(w: torch.Tensor, N: int, out_hw: Tuple[int, int], transposed: bool = False) -> int:
+    """Algorithmic MACs of the reference op (dense count, for rooflines) from its un-transformed weights
+    ([Cout, Cin/groups, kh, kw], or [Cin, Cout, 4, 4] when ``transposed``) and its output extent: one MAC per weight
+    element and output pixel; a ConvTranspose2d(k4, s2, p1) uses a quarter of its taps for each output pixel."""
+    macs = N * out_hw[0] * out_hw[1] * w.numel()
+    return macs // 4 if transposed else macs
 
 
 def choose_tile(Hq: int, Wq: int) -> Tuple[int, int]:
@@ -184,8 +191,8 @@ def plan_conv(srcs: Sequence[Tuple[Tuple[int, int, int, int, int], bool]], weigh
         assert len(srcs) == 1 and groups == 1 and tuple(w.shape[2:]) == (4, 4) and not any_up
         (_, H, W, cin, _), _ = srcs[0]
         assert w.shape[0] == cin
+        cout = w.shape[1]
         phases, Hq, Wq, out_H, out_W = 4, H, W, 2 * H, 2 * W
-        macs = N * H * W * cin * w.shape[1] * 16
     else:
         cout, cin_g, kh, kw = w.shape
         cin_total = sum(s[3] for s, _ in srcs)
@@ -203,14 +210,6 @@ def plan_conv(srcs: Sequence[Tuple[Tuple[int, int, int, int, int], bool]], weigh
                 out_hw = ((H + 2 * pad[0] - kh) // stride + 1, (W + 2 * pad[1] - kw) // stride + 1)
             out_H, out_W = out_hw
             phases, Hq, Wq = 1, out_H, out_W
-        macs = N * out_H * out_W * cout * cin_g * kh * kw
-    return _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, tuple(pad), groups, transposed, out_bf16, macs,
-                 packed_dtype)
-
-
-def _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, pad, groups, transposed, out_bf16, macs,
-          packed_dtype=torch.bfloat16):
-    cout = w.shape[1] if transposed else w.shape[0]
     cout_w = pad8(cout) if out_bf16 else cout          # channels the kernel writes
     TH, TW = choose_tile(Hq, Wq)
     if groups > 1:
@@ -230,10 +229,8 @@ def _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, pad, groups, transpo
     c_lo = 0
     for (sN, sH, sW, sC, ldc), up in srcs:
         assert sN == N
-        if transposed:
-            kc = choose_kc(sC)
-            seg = SegSpec(N, sH, sW, sC, ldc, 2, 2, 1, (-1, 0), (-1, 0), 0, -(-sC // kc), kc)
-        elif up:
+        if transposed or up:
+            # half-resolution source: 2x2 taps per output phase
             kc = choose_kc(sC)
             seg = SegSpec(N, sH, sW, sC, ldc, 2, 2, 1, (-1, 0), (-1, 0), 0, -(-sC // kc), kc)
         elif phases == 4:
@@ -241,7 +238,6 @@ def _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, pad, groups, transpo
             kc = choose_kc(sC)
             seg = SegSpec(N, sH, sW, sC, ldc, 3, 3, 2, (-1, 0), (-1, 0), 0, -(-sC // kc), kc)
         else:
-            kh, kw = w.shape[2], w.shape[3]
             cg = sC // groups
             kc = choose_kc(cg if groups > 1 else sC, kh * kw)
             seg = SegSpec(N, sH, sW, sC, ldc, kh, kw, stride, (-pad[0], -pad[0]), (-pad[1], -pad[1]),
@@ -288,8 +284,11 @@ def _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, pad, groups, transpo
         if (sg.mul == 1 and sg.kh * sg.kw >= 4 and sg.kh <= 7 and sg.kw <= 7 and b_bytes <= HALO_B_BYTES
                 and Hq * Wq >= 0.75 * cover):
             halo, TH, TW = 1, 16, 8
-    if (TH != 1 and not halo and phases == 1 and not transposed and BN <= 128
-            and all(sg.kc == 64 and sg.mul == 1 and sg.kw >= 2 and (sg.c_per_tile == 0 or sg.cchunks == 1) for sg in segs)):
+
+    def wide_boxes(sg: SegSpec) -> bool:
+        """Under a row tile, the kw taps of a tap row of this segment can share one A box."""
+        return sg.kc == 64 and sg.mul == 1 and sg.kw >= 2 and BN <= 128 and (sg.c_per_tile == 0 or sg.cchunks == 1)
+    if TH != 1 and not halo and phases == 1 and not transposed and all(wide_boxes(sg) for sg in segs):
         # k x k conv over wide sources with few output channels and no resident-weight (halo) form: L2 -> shared-memory
         # traffic bounds it (every tap re-reads its A tile).  A ROW tile lets the kw taps of a tap row share one box
         # (wide boxes below: 3x less A traffic), which pays even when the row does not fill the 128 MMA rows:
@@ -307,15 +306,13 @@ def _plan(srcs, w, phases, N, Hq, Wq, out_H, out_W, stride, pad, groups, transpo
     if TH == 1 and not halo:
         # activation-traffic saver for L2-bound shapes: the B stage then holds kw weight tiles
         for sg in segs:
-            if (sg.kc == 64 and sg.mul == 1 and sg.kw >= 2 and TW + sg.kw - 1 <= 136 and BN <= 128
-                    and (sg.c_per_tile == 0 or sg.cchunks == 1)):
+            if wide_boxes(sg) and TW + sg.kw - 1 <= 136:
                 sg.wide = 1
-    geom = ConvGeom(segs, phases, N, Hq, Wq, TH, TW, BN, n_tiles_n, cout_per_tile, cout_w, Ktot, out_H, out_W,
-                    macs, halo)
+    geom = ConvGeom(segs, phases, N, Hq, Wq, TH, TW, BN, n_tiles_n, cout_per_tile, cout_w, Ktot, out_H, out_W, halo)
     return geom, packed
 
 
-def pixel_pack_factor(src_cps: Sequence[int], W: int, kw: int, cout_p: int) -> int:
+def pixel_pack_factor(src_cps: Sequence[int], W: int, kw: int, cout_p: int, max_f: int = 8) -> int:
     """Pixels packed along W per GEMM row for narrow tensors (0 = do not pack).  A pixel of a
     16-channel tensor is a 32-byte TMA row; packing f adjacent pixels into one f*C-channel
     "super pixel" (same memory, different view) gives 128-byte rows and an MMA N of f*Cout."""
@@ -323,7 +320,7 @@ def pixel_pack_factor(src_cps: Sequence[int], W: int, kw: int, cout_p: int) -> i
     if cmax > 32:
         return 0
     f = 64 // cmax
-    while f > 1 and (W % f or kw > f + 1 or f * cout_p > 256):
+    while f > 1 and (f > max_f or W % f or kw > f + 1 or f * cout_p > 256):
         f //= 2
     return f if f > 1 else 0
 
@@ -355,6 +352,16 @@ def pack_conv_weights(w: torch.Tensor, b: Optional[torch.Tensor], src_cs: Sequen
         for q in range(f):
             bp[q * cout_store:q * cout_store + cout] = b.detach().float().cpu()
     return wp, bp
+
+
+def plan_pixel_packed(srcs: Sequence[Act], w: torch.Tensor, b: Optional[torch.Tensor], f: int, pad: Tuple[int, int],
+                      cout_store: int, **kw) -> Tuple[ConvGeom, torch.Tensor, torch.Tensor]:
+    """Plan a stride-1 "same" conv over NHWC activations on their f-pixel packed view (pixel_pack_factor).  Returns
+    (geometry, packed weights, bias rows); ``kw`` goes to plan_conv."""
+    wp, bp = pack_conv_weights(w, b, [a.C for a in srcs], [a.Cp for a in srcs], f, pad[1], cout_store)
+    spec = [((a.N, a.H, a.W // f, f * a.Cp, f * a.Cp), False) for a in srcs]
+    geom, packed = plan_conv(spec, wp, pad=(pad[0], 1 if w.shape[3] > 1 else 0), **kw)
+    return geom, packed, pad_bias(bp, geom, f * cout_store)
 
 
 def d2s_weights(w: torch.Tensor, b: Optional[torch.Tensor], transposed: bool, cout_store: int) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -403,13 +410,12 @@ class ConvPlan:
 
     def __init__(self, geom: ConvGeom, packed: torch.Tensor, bias: torch.Tensor, seg_tensors: Sequence[torch.Tensor],
                  out: torch.Tensor, out_mode: str = 'bf16_nhwc', act: str = 'none',
-                 res: Optional[torch.Tensor] = None, res_mode: str = 'none', out_c_off: int = 0,
-                 per_image_weights: bool = False, name: str = '', out_pack: int = 1,
-                 out_ldc: Optional[int] = None, d2s: int = 0,
+                 res: Optional[torch.Tensor] = None, res_mode: str = 'none', per_image_weights: bool = False,
+                 name: str = '', out_pack: int = 1, out_ldc: Optional[int] = None, d2s: int = 0,
                  head: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None):
         """head: (weight fp32 [classes][cmid], bias fp32 [classes], conv bias fp32 [cmid]) of a 1x1 segmentation head
         fused into the epilogue (octseg.h, `head_classes`): `out` is then the head's NCHW output and the conv's own
-        output is never stored."""
+        output is never stored.  The descriptor's `out_c_off` stays 0: the output starts at channel 0."""
         lib = _lib.load()
         dev = out.device
         self.geom, self.name = geom, name
@@ -436,7 +442,6 @@ class ConvPlan:
         d.out, d.out_mode = out.data_ptr(), _lib.OUT[out_mode]
         d.out_H, d.out_W = geom.out_H, geom.out_W
         d.out_ldc = out_ldc if out_ldc is not None else (out.shape[-1] if out_mode == 'bf16_nhwc' else out.shape[1])
-        d.out_c_off = out_c_off
         d.out_pack = out_pack
         d.d2s = d2s
         d.halo = geom.halo

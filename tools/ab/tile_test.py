@@ -23,7 +23,7 @@ def run(srcs, cout, k, tile=None, tag=''):
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / 10
     print(json.dumps(dict(tag=tag, tile=(geom.TH, geom.TW), BN=geom.BN, halo=geom.halo, wide=[s.wide for s in geom.segs], ms=round(ms, 4),
-                          tflops=round(2 * geom.macs / ms / 1e9, 1))), flush=True)
+                          tflops=round(2 * C.dense_macs(w, N, (geom.out_H, geom.out_W)) / ms / 1e9, 1))), flush=True)
 for tile in (None, (1, 112), (2, 56), (1, 128), (8, 16)):
     run([(168, 224, 224)], 64, 3, tile, 'vv dec2 skip 168->64 @224')
 for tile in (None, (1, 112), (1, 128)):

@@ -53,7 +53,7 @@ def main():
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / reps
-        tflops = 2 * geom.macs / (ms * 1e-3) / 1e12
+        tflops = 2 * C.dense_macs(w, n, (geom.out_H, geom.out_W)) / (ms * 1e-3) / 1e12
         executed = 2.0 * n * geom.phases * geom.Hq * geom.Wq * geom.n_tiles_n * geom.BN * geom.Ktot / (ms * 1e-3) / 1e12
         r = dict(layer=name, batch=n, ms=round(ms, 4), tflops_algorithmic=round(tflops, 1),
                  tflops_executed=round(executed, 1), tile=(geom.TH, geom.TW), BN=geom.BN, ntn=geom.n_tiles_n,

@@ -27,6 +27,7 @@ def main():
         spec = [((n, s[1], s[2], s[0], C.pad8(s[0])), False) for s in srcs]
         w = torch.randn(cout, sum(s[0] for s in srcs), k, k) * 0.05
         geom, packed = C.plan_conv(spec, w, pad=(k // 2, k // 2))
+        macs = C.dense_macs(w, n, (geom.out_H, geom.out_W))
         bias = C.pad_bias(torch.zeros(cout), geom, cout)
         seg_t = [torch.randn(n, s[1], s[2], C.pad8(s[0]), device='cuda').to(torch.bfloat16) for s in srcs]
         out = torch.empty(n, geom.out_H, geom.out_W, geom.Cout, dtype=torch.bfloat16, device='cuda')
@@ -44,7 +45,7 @@ def main():
         bytes_io = sum(t.numel() * 2 for t in seg_t) + out.numel() * 2
         tiles = geom.phases * geom.N * -(-geom.Hq // geom.TH) * -(-geom.Wq // geom.TW) * geom.n_tiles_n
         print(json.dumps(dict(layer=name, ms=round(ms, 4), TBps=round(bytes_io / ms / 1e9, 2),
-                              tflops=round(2 * geom.macs / ms / 1e9, 1), tile=(geom.TH, geom.TW), BN=geom.BN,
+                              tflops=round(2 * macs / ms / 1e9, 1), tile=(geom.TH, geom.TW), BN=geom.BN,
                               ntn=geom.n_tiles_n, kc=[s.kc for s in geom.segs], tiles=tiles,
                               clk_per_tile_per_sm=round(ms * 1e-3 * 1.9e9 / (tiles / 148)))), flush=True)
 

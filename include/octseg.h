@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define OCTSEG_ABI_VERSION 3
+#define OCTSEG_ABI_VERSION 4
 
 enum {
   OCTSEG_OK = 0,
@@ -132,6 +132,22 @@ typedef struct octseg_conv_plan octseg_conv_plan;
 int octseg_conv_plan_create(const octseg_conv_desc* desc, octseg_conv_plan** plan);
 int octseg_conv_plan_destroy(octseg_conv_plan* plan);
 int octseg_conv_run(const octseg_conv_plan* plan, void* stream);
+
+/* What octseg_conv_plan_create decided for a plan (read-only; for tests and diagnostics).  The struct is used
+   through its tag: the function below has the same name. */
+struct octseg_conv_plan_info {
+  int32_t grid;          /* persistent CTAs launched: min(total_tiles, SMs)                           */
+  int32_t total_tiles;   /* phases * N * tiles_h * tiles_w * n_tiles_n                                */
+  int32_t n_acc;         /* accumulators in the TMEM ring: min(8, 512 / BN)                           */
+  int32_t nstages;       /* shared-memory pipeline stages                                             */
+  int32_t use_tma_store; /* bf16 output leaves through TMA stores (else direct stores)                */
+  int32_t out_grouped;   /* grouped conv stored through the 5-D (c, group, w, h, n) map              */
+  int32_t d2s_tma;       /* depth-to-space output stored through TMA                                  */
+  int32_t own_spatial;   /* a CTA takes whole spatial tiles, all their channel tiles back to back     */
+  int32_t halo;          /* halo-tile mode                                                            */
+  int32_t wide;          /* some segment loads wide (one box per tap row) A boxes                     */
+};
+int octseg_conv_plan_info(const octseg_conv_plan* plan, struct octseg_conv_plan_info* info);
 
 /* ------------------------------------------------------------------------------------------
  * CUDA-core kernels for the HBM-bound / tiny-K layers.

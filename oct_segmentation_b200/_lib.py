@@ -20,7 +20,7 @@ OUT = {'bf16_nhwc': 0, 'f32_nchw': 1, 'u8_nchw': 2}
 # every symbol include/octseg.h declares; tests check the .so exports all of them
 EXPORTS = [
     'octseg_last_error', 'octseg_abi_version', 'octseg_sm_count',
-    'octseg_conv_plan_create', 'octseg_conv_plan_destroy', 'octseg_conv_run',
+    'octseg_conv_plan_create', 'octseg_conv_plan_destroy', 'octseg_conv_run', 'octseg_conv_plan_info',
     'octseg_stem_pack', 'octseg_maxpool3x3s2', 'octseg_dwconv', 'octseg_se_hidden',
     'octseg_se_gate', 'octseg_se_scale_weights', 'octseg_preprocess_resize_bgr', 'octseg_postprocess',
     'octseg_radial_thickness', 'octseg_overlay', 'octseg_preprocess_resize_gray',
@@ -52,6 +52,12 @@ class ConvDesc(C.Structure):
     ]
 
 
+class ConvPlanInfo(C.Structure):
+    """struct octseg_conv_plan_info: what octseg_conv_plan_create decided for a plan."""
+    _fields_ = [(n, C.c_int32) for n in ('grid', 'total_tiles', 'n_acc', 'nstages', 'use_tma_store', 'out_grouped',
+                                         'd2s_tma', 'own_spatial', 'halo', 'wide')]
+
+
 class OctsegError(RuntimeError):
     pass
 
@@ -75,6 +81,7 @@ def load() -> C.CDLL:
     lib.octseg_conv_plan_create.argtypes = [C.POINTER(ConvDesc), C.POINTER(C.c_void_p)]
     lib.octseg_conv_plan_destroy.argtypes = [C.c_void_p]
     lib.octseg_conv_run.argtypes = [C.c_void_p, C.c_void_p]
+    lib.octseg_conv_plan_info.argtypes = [C.c_void_p, C.POINTER(ConvPlanInfo)]
     lib.octseg_stem_pack.argtypes = [
         C.c_void_p, C.c_int32, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int32,
         C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_void_p, C.c_void_p]
@@ -110,7 +117,7 @@ def load() -> C.CDLL:
     for name in EXPORTS:
         if name not in ('octseg_last_error',):
             getattr(lib, name).restype = C.c_int
-    if lib.octseg_abi_version() != 3:
+    if lib.octseg_abi_version() != 4:
         raise OctsegError('liboctseg.so ABI version mismatch')
     _lib = lib
     return lib

@@ -1368,6 +1368,23 @@ extern "C" int octseg_conv_plan_destroy(octseg_conv_plan* plan) {
   return OCTSEG_OK;
 }
 
+extern "C" int octseg_conv_plan_info(const octseg_conv_plan* plan, struct octseg_conv_plan_info* info) {
+  if (!plan || !info) return fail(OCTSEG_EINVAL, "null argument");
+  const ConvKParams& kp = plan->kp;
+  info->grid = plan->grid;
+  info->total_tiles = kp.total_tiles;
+  info->n_acc = kp.n_acc;
+  info->nstages = kp.nstages;
+  info->use_tma_store = kp.use_tma_store;
+  info->out_grouped = kp.out_grouped;
+  info->d2s_tma = kp.d2s_tma;
+  info->own_spatial = kp.own_spatial;
+  info->halo = kp.halo;
+  info->wide = 0;
+  for (int s = 0; s < kp.nseg; ++s) info->wide |= kp.seg[s].wide;
+  return OCTSEG_OK;
+}
+
 #ifdef OCTSEG_TRACE
 extern "C" int octseg_debug_trace(unsigned long long* h_out) {
   OCTSEG_CUDA(cudaMemcpyFromSymbol(h_out, octseg::g_trace, sizeof(unsigned long long) * kTraceEvents * kTraceTiles));

@@ -458,6 +458,12 @@ class ConvPlan:
         _lib.check(self._lib.octseg_conv_run(self._h, stream if stream is not None else _lib.stream_ptr()),
                    f'conv_run({self.name})')
 
+    def info(self) -> dict:
+        """The library's launch decisions for this plan (octseg_conv_plan_info): grid, tiles, ring sizes, mode flags."""
+        out = _lib.ConvPlanInfo()
+        _lib.check(self._lib.octseg_conv_plan_info(self._h, C.byref(out)), f'conv_plan_info({self.name})')
+        return {n: getattr(out, n) for n, _ in out._fields_}
+
     def __del__(self):
         h = getattr(self, '_h', None)
         if h:

@@ -17,14 +17,17 @@ from oct_segmentation_b200 import predict as pred
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_abi_4():
+    """ABI 4 added octseg_conv_plan_info; the header, the library and the binding must agree on it."""
     header = open(os.path.join(ROOT, 'include', 'octseg.h')).read()
     declared = set(re.findall(r'\b(octseg_[a-z0-9_]+)\s*\(', header))
     assert declared == set(_lib.EXPORTS), declared ^ set(_lib.EXPORTS)
+    assert 'octseg_conv_plan_info' in declared
     lib = ctypes.CDLL(_lib.LIB_PATH)
     for name in declared:
         assert hasattr(lib, name), name
-    assert _lib.load().octseg_abi_version() == 3
+    assert re.search(r'#define OCTSEG_ABI_VERSION 4\b', header)
+    assert _lib.load().octseg_abi_version() == 4
 
 
 def test_conv_plan_rejects_bad_arguments_without_a_gpu():
@@ -353,10 +356,13 @@ def test_ctypes_conv_desc_layout_matches_the_c_header(tmp_path):
         pytest.skip('no gcc')
     names = [n for n, _ in _lib.ConvDesc._fields_]
     seg_names = [n for n, _ in _lib.ConvSeg._fields_]
+    info_names = [n for n, _ in _lib.ConvPlanInfo._fields_]
     src = ['#include <stddef.h>', '#include <stdio.h>', '#include "octseg.h"', 'int main(void) {',
-           '  printf("sizeof %zu %zu\\n", sizeof(octseg_conv_desc), sizeof(octseg_conv_seg));']
+           '  printf("sizeof %zu %zu %zu\\n", sizeof(octseg_conv_desc), sizeof(octseg_conv_seg),',
+           '         sizeof(struct octseg_conv_plan_info));']
     src += [f'  printf("d {n} %zu\\n", offsetof(octseg_conv_desc, {n}));' for n in names]
     src += [f'  printf("s {n} %zu\\n", offsetof(octseg_conv_seg, {n}));' for n in seg_names]
+    src += [f'  printf("i {n} %zu\\n", offsetof(struct octseg_conv_plan_info, {n}));' for n in info_names]
     src += ['  return 0;', '}']
     c = tmp_path / 'layout.c'
     c.write_text('\n'.join(src))
@@ -364,10 +370,11 @@ def test_ctypes_conv_desc_layout_matches_the_c_header(tmp_path):
     inc = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'include')
     subprocess.run(['gcc', '-I', inc, '-o', str(exe), str(c)], check=True)
     out = subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.split('\n')
-    assert out[0] == f'sizeof {ctypes.sizeof(_lib.ConvDesc)} {ctypes.sizeof(_lib.ConvSeg)}'
+    assert out[0] == (f'sizeof {ctypes.sizeof(_lib.ConvDesc)} {ctypes.sizeof(_lib.ConvSeg)} '
+                      f'{ctypes.sizeof(_lib.ConvPlanInfo)}')
     for line in out[1:]:
         if not line:
             continue
         kind, name, off = line.split()
-        cls = _lib.ConvDesc if kind == 'd' else _lib.ConvSeg
+        cls = {'d': _lib.ConvDesc, 's': _lib.ConvSeg, 'i': _lib.ConvPlanInfo}[kind]
         assert getattr(cls, name).offset == int(off), (kind, name)
